@@ -2,6 +2,11 @@
 """bench.py -- SGD samples/sec on RCV1-shaped synthetic sparse data (BASELINE.json's metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch 256] [--mode sync]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR writes, after the timed steps, what the timed leg computed in its last bench step: sync mode
+weights.npy (the final weights) and losses.npy (the loss of each SGD step); async mode master_weights.npy.  The inputs
+depend only on the arguments (seeded synthetic rows and batch draws), so sync outputs of two builds compare one to one.
 
 Workload (BASELINE.json configs[1]/[2]): sync mode, RCV1-shaped synthetic rows (47 236 features, 700 000
 rows of which the first 80 % train -- Main.scala:52 --, ~0.2 % non-zeros), batch 256 per GPU, lambda 1e-5,
@@ -74,7 +79,13 @@ def parse():
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip sweep / async / parity / rpc_seam / e2e_fit sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last bench step to DIR/<name>.npy (fp64)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs: the reference arm sizes its sample by elapsed time, its outputs are not reproducible")
     if a.batch is None:
         a.batch = 256 if a.mode == "sync" else 1        # BASELINE.json configs[1]/[2] and configs[3]
     return a
@@ -225,6 +236,21 @@ def draw_batches(rng, lo: int, hi: int, batch: int, n_steps: int) -> np.ndarray:
     for s in range(n_steps):
         out[s] = lo + rng.choice(hi - lo, size=batch, replace=False)
     return out
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, fp64, so that two builds run with the same arguments (hence the same
+    seeded inputs) can be compared output for output."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed {DUMP_MAX_BYTES}; use fewer --sgd-steps")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def make_oracle(data, d):
@@ -519,6 +545,8 @@ def bench_async(args, ctx, data, n_train, d, group, rank, local_rank, world):
     value = samples_total / (ms_dev * 1e-3)
     e2e_value = samples_total / wall
     w_master = ctx.async_master_weights() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:      # Hogwild: the update order, hence the weights, differ from run to run
+        dump_outputs(args.dump_outputs, {"master_weights": w_master})
     hbm_peak, peak_src = peaks()
     mean_bytes = data.algorithmic_bytes() / data.n_rows
     achieved = (args.steps * U * B * mean_bytes) / (ms_dev * 1e-3) / 1e9     # per GPU
@@ -667,6 +695,8 @@ def main():
     value = samples_total / (ms * 1e-3)
     w_after = ctx.get_weights()
     last_losses = ctx.read_losses(S)
+    if rank == 0 and args.dump_outputs:      # replicas are bit-identical and the losses cover every worker's samples
+        dump_outputs(args.dump_outputs, {"weights": w_after, "losses": last_losses})
 
     # ---- leg 2: end to end through the C-ABI call with host buffers (e2e) --------------------------------
     ctx.set_weights(np.zeros(data.dim))
