@@ -277,6 +277,84 @@ class MasterSync(Master):
             if on_epoch:
                 on_epoch(epoch, {"loss": tl, "acc": ta, "test_loss": vl, "test_acc": va})
 
+    def fit_models(self, initial_weights: np.ndarray, max_epochs: int, batch_size: int, lambdas: Sequence[float],
+                   learning_rates: Sequence[float], stopping_criterion: EarlyStopping,
+                   split_strategy: Split = SplitStrategy.vanilla, *,
+                   on_epoch: Optional[Callable[[int, List[Optional[dict]]], None]] = None) -> List[GradState]:
+        """`fit` for several (lambda, learning rate) settings at once: one SparseSVM(lambdas[m]) trained with
+        learning_rates[m] per setting, all on the same batch draws, as a model set on the device (one kernel per run of
+        equal-count steps for all models).  Model m's GradState and history are what `fit(initial_weights, max_epochs,
+        batch_size, learning_rates[m], stopping_criterion, split_strategy)` returns on a master whose model is
+        SparseSVM(lambdas[m]) with the same seed: each model stops (is frozen) at the epoch its own test losses stop it.
+        One GPU, one worker per step.  Sets `self.histories` (one dict per model, the keys of `fit`'s `self.history`)."""
+        from ..native import MAX_MODELS
+        lambdas = [float(x) for x in lambdas]
+        learning_rates = [float(x) for x in learning_rates]
+        M = len(lambdas)
+        if len(learning_rates) != M or not 1 <= M <= MAX_MODELS:
+            raise ValueError(f"fit_models: need 1 to {MAX_MODELS} (lambda, learning rate) pairs, got {M} and "
+                             f"{len(learning_rates)}")
+        if self.group.world != 1:
+            raise ValueError("fit_models: model sets run on one GPU (process group of size 1)")
+        groups = split_strategy(self.n_train, 1)
+        if len(groups) != 1:
+            raise ValueError("fit_models: model sets take one worker per step")
+        w0 = np.asarray(initial_weights, dtype=np.float64)
+        self.ctx.models_set(lambdas, learning_rates, w0)
+        states = [GradState.start_state(w0) for _ in range(M)]
+        hist = [{"losses": [], "test_losses": [], "accs": [], "test_accs": []} for _ in range(M)]  # newest first
+        done: List[Optional[GradState]] = [None] * M
+        self.step_losses: List[np.ndarray] = []
+        n_train, n_test = self.n_train, self.n_test
+        epoch = 0
+        from concurrent.futures import ThreadPoolExecutor
+        prefetch = ThreadPoolExecutor(1) if self.jvm is None else None
+        pending = None
+        try:
+            while True:
+                for m in range(M):                                                    # Master.scala:154,166, per model
+                    if done[m] is None and (epoch >= max_epochs or stopping_criterion(hist[m]["test_losses"])):
+                        done[m] = states[m].finish(hist[m]["losses"][0])
+                active = np.array([d is None for d in done])
+                if not active.any():
+                    break
+                steps = pending.result() if pending is not None else self.draw_epoch(groups, batch_size)
+                pending = None
+                if not isinstance(steps, EpochDraw):
+                    steps = EpochDraw.from_steps(steps)
+                if prefetch is not None and epoch + 1 < max_epochs:
+                    pending = prefetch.submit(self.draw_epoch, groups, batch_size, self._epochs_drawn)
+                counts = steps.counts[:, 0]
+                if counts.size and (counts == 0).any():
+                    raise ValueError("Cannot sum an empty list of vectors")       # Vec.scala:129 via Master.scala:187 (Q7)
+                n_steps = counts.shape[0]
+                bounds = [0, *(np.flatnonzero(counts[1:] != counts[:-1]) + 1).tolist(), n_steps]
+                for i, j in zip(bounds[:-1], bounds[1:]):
+                    if j == i:
+                        continue
+                    c = int(counts[i])
+                    flat = np.ascontiguousarray(steps.ids[i:j, 0, :c]).reshape(-1)
+                    self.step_losses.append(self.ctx.models_steps(flat, c, j - i, active=active))
+                epoch += 1
+                weights = self.ctx.models_get_weights()
+                report: List[Optional[dict]] = [None] * M
+                for m in np.flatnonzero(active).tolist():
+                    h, cr, n2 = self.ctx.models_eval_counts(m, 0, n_train)                     # Master.scala:206-207
+                    th, tc, _ = self.ctx.models_eval_counts(m, n_train, n_train + n_test)      # Master.scala:208-209
+                    tl, ta = lambdas[m] * n2 + h / n_train, cr / n_train
+                    vl, va = lambdas[m] * n2 + th / n_test, tc / n_test
+                    for k, v in (("losses", tl), ("accs", ta), ("test_losses", vl), ("test_accs", va)):
+                        hist[m][k].insert(0, v)
+                    states[m] = states[m].replace_grad(weights[m].copy())                  # Master.scala:205
+                    report[m] = {"loss": tl, "acc": ta, "test_loss": vl, "test_acc": va}
+                if on_epoch:
+                    on_epoch(epoch, report)
+        finally:
+            if prefetch is not None:
+                prefetch.shutdown(wait=True)
+        self.histories = [{k: v[::-1] for k, v in h.items()} for h in hist]
+        return done
+
 
 class MasterAsync(Master):
     """core/MasterAsync.scala -- Hogwild: every worker runs its loop on its GPU and pushes deltas into every peer

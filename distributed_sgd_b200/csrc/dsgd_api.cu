@@ -7,6 +7,8 @@
 #include <nccl.h>  // types only: the library itself is bound at run time (see nccl_api)
 
 #include <algorithm>
+#include <cmath>
+#include <limits>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -17,6 +19,7 @@
 #include "dsgd_persistent.cuh"
 #include "dsgd_stream.cuh"
 #include "dsgd_async.cuh"
+#include "dsgd_models.cuh"
 #include <cstdlib>
 
 using namespace dsgd;
@@ -105,6 +108,18 @@ struct dsgd_ctx {
   int64_t x_steps_run = 0;  // SGD steps run by the fused kernel so far (dsgd_xchg_stats)
   unsigned long long *x_llw = nullptr;  // this rank's weights in LL form, two parities
   unsigned long long *x_stats = nullptr;  // [0] value words, [1] bitmap words pushed to each peer so far; [2] SGD steps of those launches
+
+  // model set (dsgd_models_*): resident weights of every model and the model-set kernel's buffers
+  int32_t ms_n = 0;
+  std::vector<double> ms_lambda, ms_lr;
+  double *ms_w = nullptr;               // [ms_n][dim]
+  double2 *ms_rec = nullptr;            // [ms_n][3][dim]: rotating {W, g} records
+  unsigned long long *ms_acc = nullptr; // [3][ms_n][kAccStride]
+  unsigned *ms_hinge = nullptr;         // [n_steps][active models]
+  double *ms_losses = nullptr;
+  int64_t ms_hinge_cap = 0, ms_losses_cap = 0;
+  unsigned *ms_bar = nullptr;           // [0]: grid barrier counter, [1]: abort flag
+  bool ms_ready = false;
 
   // sampled per-launch timing of the gradient kernel
   int32_t prof_every = 0;
@@ -286,7 +301,7 @@ extern "C" int dsgd_destroy(dsgd_ctx *ctx) {
   void *ptrs[] = {ctx->rp16, ctx->pairs, ctx->label, ctx->yabs, ctx->w, ctx->g, ctx->d, ctx->w_req, ctx->w32, ctx->w32_req, ctx->n_exact, ctx->scal,
                   ctx->cnt, ctx->partial, ctx->out2, ctx->gsum, ctx->p_wbuf[0], ctx->p_wbuf[1], ctx->p_gbuf[0],
                   ctx->p_gbuf[1], ctx->p_gbuf[2], ctx->p_rec[0], ctx->p_rec[1], ctx->p_rec[2], ctx->p_acc, ctx->p_hinge, ctx->p_bar, ctx->x_stats, ctx->samples,
-                  ctx->losses, ctx->preds};
+                  ctx->losses, ctx->preds, ctx->ms_w, ctx->ms_rec, ctx->ms_acc, ctx->ms_hinge, ctx->ms_losses, ctx->ms_bar};
   for (void *p : ptrs) if (p) cudaFree(p);
   if (ctx->ev0) cudaEventDestroy(ctx->ev0);
   if (ctx->ev1) cudaEventDestroy(ctx->ev1);
@@ -545,8 +560,9 @@ extern "C" int dsgd_stage_samples(dsgd_ctx *ctx, const int32_t *samples, int64_t
 }
 
 // weights to use for a request: NULL -> resident; else copy into w_req and compute its scalars
+// (w_on_device: w is a device pointer, e.g. a model of the set)
 static int request_weights(dsgd_ctx *ctx, const double *w, const double **w_dev, const double **c_dev,
-                           const double **nrm_dev, const float **w32_dev = nullptr) {
+                           const double **nrm_dev, const float **w32_dev = nullptr, bool w_on_device = false) {
   CU(cudaSetDevice(ctx->device));  // every request path passes here: a caller thread may have another device current
   if (!w) {
     *w_dev = ctx->w; *c_dev = ctx->scal + kScalC; *nrm_dev = ctx->scal + kScalNrm2;
@@ -554,7 +570,8 @@ static int request_weights(dsgd_ctx *ctx, const double *w, const double **w_dev,
     return DSGD_OK;
   }
   if (w32_dev) *w32_dev = ctx->w32_req;
-  CU(cudaMemcpyAsync(ctx->w_req, w, sizeof(double) * (size_t)ctx->dim, cudaMemcpyHostToDevice, ctx->stream));
+  CU(cudaMemcpyAsync(ctx->w_req, w, sizeof(double) * (size_t)ctx->dim,
+                     w_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, ctx->stream));
   k_prepare<1024><<<1, 1024, 0, ctx->stream>>>(ctx->w_req, ctx->d, ctx->dim, ctx->lambda, ctx->scal + kScalReqC,
                                                 ctx->scal + kScalReqNrm2);
   LAUNCHED();
@@ -673,7 +690,8 @@ extern "C" int dsgd_gradient(dsgd_ctx *ctx, const double *w, const int32_t *samp
   return DSGD_OK;
 }
 
-static int eval_impl(dsgd_ctx *ctx, const double *w, int64_t row_begin, int64_t row_end, double out[5]) {
+static int eval_impl(dsgd_ctx *ctx, const double *w, int64_t row_begin, int64_t row_end, double out[5],
+                     bool w_on_device = false) {
   NEED(ctx->pairs, DSGD_ERR_STATE, "dsgd_eval: no rows loaded");
   NEED(row_begin >= 0 && row_end <= ctx->n_rows && row_begin <= row_end, DSGD_ERR_RANGE,
        "dsgd_eval: rows [%lld,%lld) outside [0,%lld)", (long long)row_begin, (long long)row_end, (long long)ctx->n_rows);
@@ -683,7 +701,7 @@ static int eval_impl(dsgd_ctx *ctx, const double *w, int64_t row_begin, int64_t 
   const double *wd, *cd, *nd;
   const float *w32d;
   int rc;
-  if ((rc = request_weights(ctx, w, &wd, &cd, &nd, &w32d))) return rc;
+  if ((rc = request_weights(ctx, w, &wd, &cd, &nd, &w32d, w_on_device))) return rc;
   if (stream_eligible(ctx, n)) {
     if ((rc = stream_launch<false, false, true>(ctx, nullptr, row_begin, n, wd, w32d, nullptr, nullptr))) return rc;
   } else {
@@ -1436,5 +1454,167 @@ extern "C" int dsgd_async_master_weights(dsgd_ctx *ctx, double *w_out) {
   CU(cudaSetDevice(ctx->device));
   CU(cudaMemcpyAsync(w_out, m, sizeof(double) * (size_t)ctx->dim, cudaMemcpyDeviceToHost, ctx->stream2));
   CU(cudaStreamSynchronize(ctx->stream2));
+  return DSGD_OK;
+}
+
+// ---- model sets (dsgd_models.cuh): M SparseSVMs, each with its own lambda and learning rate, on the same draws ---------
+// Main.scala:68 builds ONE `new SparseSVM(config.lambda, ...)` per run and Master.fit (core/Master.scala:179-198) trains it;
+// a model set trains up to DSGD_MAX_MODELS of them in one persistent kernel per call.  One GPU, one worker per step.
+static_assert(kMaxModels == DSGD_MAX_MODELS, "model-set cap");
+constexpr int kMCons = 8, kMUpd = 8, kMStages = 4, kMStagePairs = 2560, kMMaxChunks = 128;
+using MSmem = ModelsSmem<kMCons, kMUpd, kMStages, kMStagePairs, kMMaxChunks>;
+#define DSGD_MODELS_KERNEL k_models_persistent<kMCons, kMUpd, kMStages, kMStagePairs, kMMaxChunks>
+
+static int models_shape_ok(dsgd_ctx *ctx, const char *who) {
+  NEED(!(ctx->flags & DSGD_FLAG_ASYNC), DSGD_ERR_STATE, "%s: ctx is in async mode", who);
+  NEED(ctx->world == 1, DSGD_ERR_STATE, "%s: model sets run on one GPU (world is %d)", who, ctx->world);
+  const int32_t k_total = ctx->k_total > 0 ? ctx->k_total : ctx->world;
+  NEED(ctx->n_local == 1 && k_total == 1, DSGD_ERR_STATE, "%s: model sets take one worker per step (n_local %d, k_total %d)",
+       who, ctx->n_local, k_total);
+  return DSGD_OK;
+}
+
+static void models_free(dsgd_ctx *ctx) {
+  void *ptrs[] = {ctx->ms_w, ctx->ms_rec, ctx->ms_acc};
+  for (void *q : ptrs) if (q) cudaFree(q);
+  ctx->ms_w = nullptr; ctx->ms_rec = nullptr; ctx->ms_acc = nullptr;
+  ctx->ms_n = 0;
+  ctx->ms_lambda.clear(); ctx->ms_lr.clear();
+}
+
+extern "C" int dsgd_models_set(dsgd_ctx *ctx, int32_t n_models, const double *lambda, const double *lr, const double *w0) {
+  if (!ctx) return DSGD_ERR_INVALID;
+  int rc = models_shape_ok(ctx, "dsgd_models_set");
+  if (rc) return rc;
+  NEED(n_models >= 0 && n_models <= DSGD_MAX_MODELS, DSGD_ERR_INVALID, "dsgd_models_set: n_models %d outside [0,%d]", n_models,
+       DSGD_MAX_MODELS);
+  NEED(n_models == 0 || (lambda && lr), DSGD_ERR_INVALID, "dsgd_models_set: lambda / lr is NULL");
+  for (int32_t m = 0; m < n_models; ++m) {
+    NEED(std::isfinite(lambda[m]) && lambda[m] >= 0.0, DSGD_ERR_INVALID, "dsgd_models_set: lambda[%d] = %g is not a finite non-negative number", m, lambda[m]);
+    NEED(std::isfinite(lr[m]), DSGD_ERR_INVALID, "dsgd_models_set: lr[%d] = %g is not finite", m, lr[m]);
+  }
+  CU(cudaSetDevice(ctx->device));
+  CU(cudaStreamSynchronize(ctx->stream));
+  models_free(ctx);
+  if (n_models == 0) return DSGD_OK;
+  const size_t dim = (size_t)ctx->dim;
+  CU(cudaMalloc(&ctx->ms_w, sizeof(double) * dim * (size_t)n_models));
+  CU(cudaMalloc(&ctx->ms_rec, sizeof(double2) * 3 * dim * (size_t)n_models));
+  CU(cudaMalloc(&ctx->ms_acc, sizeof(unsigned long long) * 3 * kAccStride * (size_t)n_models));
+  if (!ctx->ms_bar) CU(cudaMalloc(&ctx->ms_bar, sizeof(unsigned) * 4));
+  if (w0) CU(cudaMemcpyAsync(ctx->ms_w, w0, sizeof(double) * dim * (size_t)n_models, cudaMemcpyHostToDevice, ctx->stream));
+  else CU(cudaMemsetAsync(ctx->ms_w, 0, sizeof(double) * dim * (size_t)n_models, ctx->stream));
+  if (!ctx->ms_ready) {
+    CU(cudaFuncSetAttribute((const void *)DSGD_MODELS_KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MSmem)));
+    ctx->ms_ready = true;
+  }
+  CU(cudaStreamSynchronize(ctx->stream));
+  ctx->ms_n = n_models;
+  ctx->ms_lambda.assign(lambda, lambda + n_models);
+  ctx->ms_lr.assign(lr, lr + n_models);
+  return DSGD_OK;
+}
+
+extern "C" int dsgd_models_shape(const dsgd_ctx *ctx, int32_t *n_models, int32_t *dim) {
+  if (!ctx) return DSGD_ERR_INVALID;
+  if (n_models) *n_models = ctx->ms_n;
+  if (dim) *dim = ctx->dim;
+  return DSGD_OK;
+}
+
+extern "C" int dsgd_models_get_weights(dsgd_ctx *ctx, double *w_out) {
+  if (!ctx) return DSGD_ERR_INVALID;
+  NEED(ctx->ms_n > 0, DSGD_ERR_STATE, "dsgd_models_get_weights: no model set (dsgd_models_set)");
+  NEED(w_out, DSGD_ERR_INVALID, "dsgd_models_get_weights: w_out is NULL");
+  CU(cudaSetDevice(ctx->device));
+  CU(cudaMemcpyAsync(w_out, ctx->ms_w, sizeof(double) * (size_t)ctx->dim * (size_t)ctx->ms_n, cudaMemcpyDeviceToHost,
+                     ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  return DSGD_OK;
+}
+
+extern "C" int dsgd_models_steps(dsgd_ctx *ctx, const int32_t *samples, int64_t n_per_step, int64_t n_steps,
+                                 const uint8_t *active, double *losses_out) {
+  if (!ctx) return DSGD_ERR_INVALID;
+  int rc = models_shape_ok(ctx, "dsgd_models_steps");
+  if (rc) return rc;
+  NEED(ctx->have_d, DSGD_ERR_STATE, "dsgd_models_steps: dimSparsity not set");
+  NEED(ctx->ms_n > 0, DSGD_ERR_STATE, "dsgd_models_steps: no model set (dsgd_models_set)");
+  NEED(n_steps >= 0 && n_per_step >= 0, DSGD_ERR_INVALID, "dsgd_models_steps: bad arguments");
+  NEED(n_per_step > 0, DSGD_ERR_EMPTY, "dsgd_models_steps: empty batch (Vec.sum of an empty list throws in the reference)");
+  NEED(n_steps == 0 || samples, DSGD_ERR_INVALID, "dsgd_models_steps: samples is NULL");
+  NEED(n_steps <= INT64_MAX / n_per_step, DSGD_ERR_INVALID, "dsgd_models_steps: too many samples");
+  const int G = persist_grid(ctx, n_per_step);
+  NEED(G > 0, DSGD_ERR_INVALID, "dsgd_models_steps: %lld samples per step exceed the kernel's %d rows per SM",
+       (long long)n_per_step, kMaxRowsPerCta);
+  NEED((uint64_t)G * (uint64_t)(n_steps + 2) < (1ull << 32), DSGD_ERR_INVALID, "dsgd_models_steps: too many steps for one launch");
+  const int M = ctx->ms_n;
+  ModelsParams pp;
+  memset(&pp, 0, sizeof pp);
+  int n_act = 0;
+  for (int m = 0; m < M; ++m)
+    if (!active || active[m]) {
+      pp.id[n_act] = m;
+      pp.lambda[n_act] = ctx->ms_lambda[(size_t)m];
+      pp.lr[n_act] = ctx->ms_lr[(size_t)m];
+      ++n_act;
+    }
+  if ((rc = dsgd_stage_samples(ctx, samples, n_per_step * n_steps))) return rc;
+  if (n_steps == 0 || n_act == 0) {
+    if (losses_out)
+      for (int64_t i = 0; i < n_steps * M; ++i) losses_out[i] = std::numeric_limits<double>::quiet_NaN();
+    CU(cudaStreamSynchronize(ctx->stream));
+    return DSGD_OK;
+  }
+  if ((rc = ensure_dev(ctx, (void **)&ctx->ms_hinge, &ctx->ms_hinge_cap, n_steps * n_act, sizeof(unsigned)))) return rc;
+  if (losses_out && (rc = ensure_f64(ctx, &ctx->ms_losses, &ctx->ms_losses_cap, n_steps * n_act))) return rc;
+  pp.rp16 = ctx->rp16; pp.pairs = ctx->pairs; pp.label = ctx->label; pp.samples = ctx->samples;
+  pp.n_steps = n_steps; pp.batch = (int32_t)n_per_step; pp.dim = ctx->dim; pp.n_act = n_act;
+  pp.rec_stride = ctx->dim; pp.rec = ctx->ms_rec; pp.d = ctx->d; pp.acc = ctx->ms_acc;
+  pp.hinge = ctx->ms_hinge; pp.losses = losses_out ? ctx->ms_losses : nullptr; pp.w_res = ctx->ms_w;
+  pp.bar = ctx->ms_bar; pp.abort_flag = reinterpret_cast<int *>(ctx->ms_bar + 1);
+  pp.timeout_cycles = 4000000000ll;  // ~2 s at 1.9 GHz, as for the single-model kernel
+  CU(cudaMemsetAsync(ctx->ms_acc, 0, sizeof(unsigned long long) * 3 * kAccStride * (size_t)n_act, ctx->stream));
+  CU(cudaMemsetAsync(ctx->ms_hinge, 0, sizeof(unsigned) * (size_t)(n_steps * n_act), ctx->stream));
+  CU(cudaMemsetAsync(ctx->ms_bar, 0, sizeof(unsigned) * 4, ctx->stream));
+  // every launch starts from the resident weights of its models: several calls continue one trajectory
+  k_models_rec_init<<<dim3(cdiv(ctx->dim, 256), n_act), 256, 0, ctx->stream>>>(pp);
+  LAUNCHED();
+  void *args[] = {&pp};
+  const dim3 block((kMCons + kMUpd + 1) * 32);
+  auto *pe = prof_slot(ctx);
+  if (pe) cudaEventRecord(pe->first, ctx->stream);
+  if (ctx->grid_limit > 0) CU(cudaLaunchKernel((void *)DSGD_MODELS_KERNEL, dim3(G), block, args, sizeof(MSmem), ctx->stream));
+  else CU(cudaLaunchCooperativeKernel((void *)DSGD_MODELS_KERNEL, dim3(G), block, args, sizeof(MSmem), ctx->stream));
+  if (pe) cudaEventRecord(pe->second, ctx->stream);
+  LAUNCHED();
+  if (losses_out) {
+    std::vector<double> compact((size_t)(n_steps * n_act));
+    CU(cudaMemcpyAsync(compact.data(), ctx->ms_losses, sizeof(double) * compact.size(), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    for (int64_t s = 0; s < n_steps; ++s) {
+      int k = 0;
+      for (int m = 0; m < M; ++m)
+        losses_out[s * M + m] = (!active || active[m]) ? compact[(size_t)(s * n_act + k++)] : std::numeric_limits<double>::quiet_NaN();
+    }
+  }
+  CU(cudaStreamSynchronize(ctx->stream));
+  unsigned host[2] = {0, 0};
+  CU(cudaMemcpy(host, ctx->ms_bar, sizeof host, cudaMemcpyDeviceToHost));
+  NEED(host[1] == 0, DSGD_ERR_TIMEOUT, "model-set kernel: a device-side wait (grid barrier, stage) hit its watchdog");
+  return DSGD_OK;
+}
+
+extern "C" int dsgd_models_eval_counts(dsgd_ctx *ctx, int32_t m, int64_t row_begin, int64_t row_end, int64_t *hinge_sum,
+                                       int64_t *correct, double *norm_squared) {
+  if (!ctx) return DSGD_ERR_INVALID;
+  NEED(ctx->ms_n > 0, DSGD_ERR_STATE, "dsgd_models_eval_counts: no model set (dsgd_models_set)");
+  NEED(m >= 0 && m < ctx->ms_n, DSGD_ERR_INVALID, "dsgd_models_eval_counts: model %d outside [0,%d)", m, ctx->ms_n);
+  double out[5];
+  int rc = eval_impl(ctx, ctx->ms_w + (size_t)m * (size_t)ctx->dim, row_begin, row_end, out, true);
+  if (rc) return rc;
+  if (hinge_sum) *hinge_sum = (int64_t)out[2];
+  if (correct) *correct = (int64_t)out[3];
+  if (norm_squared) *norm_squared = out[4];
   return DSGD_OK;
 }

@@ -34,6 +34,14 @@ object DsgdNative {
   @native def xchgStats(ctx: Long, out: Array[Long]): Int
   @native def setWorkers(ctx: Long, counts: Array[Int], kTotal: Int): Int
   @native def syncSteps(ctx: Long, samples: Array[Int], nPerStep: Long, nSteps: Long, lr: Double, losses: Array[Double]): Int
+  // model sets: one SparseSVM per (lambda(m), lr(m)) on the same draws; weights / losses are model-major / step-major
+  @native def modelsSet(ctx: Long, lambda: Array[Double], lr: Array[Double], w0: Array[Double]): Int  // w0 == null: zeros
+  @native def modelsShape(ctx: Long, out: Array[Int]): Int             // out(0) models, out(1) dim
+  @native def modelsGetWeights(ctx: Long, out: Array[Double]): Int     // models * dim
+  @native def modelsSteps(ctx: Long, samples: Array[Int], nPerStep: Long, nSteps: Long, active: Array[Byte],
+                          losses: Array[Double]): Int                  // active == null: all; losses: nSteps * models
+  @native def modelsEvalCounts(ctx: Long, m: Int, rowBegin: Long, rowEnd: Long, hingeCorrect: Array[Long],
+                               normSquared: Array[Double]): Int
   // async (Hogwild) mode
   @native def asyncHostMaster(ctx: Long, w0: Array[Double]): Int
   @native def ipcExport(ctx: Long, which: Int, handle: Array[Byte]): Int

@@ -192,6 +192,77 @@ FN(syncSteps)(JNIEnv *env, jobject self, jlong h, jintArray samples, jlong n_per
   return rc;
 }
 
+/* ---- model sets: one SparseSVM per (lambda, lr) setting on the same draws (Main.scala:68; core/Master.scala:179-198).
+ *      Every Java array is checked against the set's n_models, dim and n_steps * n_models before the ABI sees it; the
+ *      products are formed in 64 bits after their factors are bounded. */
+static int models_shape(jlong h, int64_t *n_models, int64_t *dim) {
+  int32_t n = 0, d = 0;
+  int rc = dsgd_models_shape(CTX(h), &n, &d);
+  *n_models = n; *dim = d;
+  return rc;
+}
+FN(modelsShape)(JNIEnv *env, jobject self, jlong h, jintArray out) {   /* out(0) n_models, (1) dim */
+  buf_t b = out_Int(env, out);
+  int rc = b.bad ? DSGD_ERR_NOMEM : (b.n < 2 ? DSGD_ERR_INVALID : dsgd_models_shape(CTX(h), (int32_t *)b.p, (int32_t *)b.p + 1));
+  back_Int(env, out, b, rc);
+  return rc;
+}
+FN(modelsSet)(JNIEnv *env, jobject self, jlong h, jdoubleArray lambda, jdoubleArray lr, jdoubleArray w0) {
+  int64_t n_old = 0, dim = 0;
+  int rc = models_shape(h, &n_old, &dim);
+  if (rc != DSGD_OK) return rc;
+  const jsize n = lambda ? (*env)->GetArrayLength(env, lambda) : 0;
+  const jsize n_lr = lr ? (*env)->GetArrayLength(env, lr) : 0;
+  if (n > DSGD_MAX_MODELS || n_lr != n) return DSGD_ERR_INVALID;
+  if (w0 && (int64_t)(*env)->GetArrayLength(env, w0) != (int64_t)n * dim) return DSGD_ERR_INVALID;
+  buf_t bl = in_Double(env, lambda), br = in_Double(env, lr), bw = in_Double(env, w0);
+  rc = DSGD_ERR_NOMEM;
+  if (!(bl.bad | br.bad | bw.bad)) rc = dsgd_models_set(CTX(h), (int32_t)n, bl.p, br.p, bw.p);
+  free(bl.p); free(br.p); free(bw.p);
+  return rc;
+}
+FN(modelsGetWeights)(JNIEnv *env, jobject self, jlong h, jdoubleArray out) {   /* out: n_models * dim, model-major */
+  int64_t n = 0, dim = 0;
+  int rc = models_shape(h, &n, &dim);
+  if (rc != DSGD_OK) return rc;
+  if (!out || (int64_t)(*env)->GetArrayLength(env, out) != n * dim) return DSGD_ERR_INVALID;
+  buf_t b = out_Double(env, out);
+  rc = b.bad ? DSGD_ERR_NOMEM : dsgd_models_get_weights(CTX(h), b.p);
+  back_Double(env, out, b, rc);
+  return rc;
+}
+FN(modelsSteps)(JNIEnv *env, jobject self, jlong h, jintArray samples, jlong n_per_step, jlong n_steps, jbyteArray active,
+                jdoubleArray losses) {
+  int64_t n = 0, dim = 0;
+  int rc = models_shape(h, &n, &dim);
+  if (rc != DSGD_OK) return rc;
+  if (n_per_step < 0 || n_steps < 0) return DSGD_ERR_INVALID;
+  if (n_steps > 0 && n_per_step > INT64_MAX / n_steps) return DSGD_ERR_INVALID;
+  const int64_t n_ids = n_per_step * n_steps;   /* n <= DSGD_MAX_MODELS: n_steps * n overflows only for absurd n_steps */
+  if (n > 0 && n_steps > INT64_MAX / n) return DSGD_ERR_INVALID;
+  if ((int64_t)(samples ? (*env)->GetArrayLength(env, samples) : 0) < n_ids) return DSGD_ERR_INVALID;
+  if (active && (int64_t)(*env)->GetArrayLength(env, active) != n) return DSGD_ERR_INVALID;
+  if (losses && (int64_t)(*env)->GetArrayLength(env, losses) < n_steps * n) return DSGD_ERR_INVALID;
+  buf_t bs = in_Int(env, samples), ba = in_Byte(env, active), bl = out_Double(env, losses);
+  rc = DSGD_ERR_NOMEM;
+  if (!(bs.bad | ba.bad | bl.bad))
+    rc = dsgd_models_steps(CTX(h), bs.p, n_per_step, n_steps, (const uint8_t *)ba.p, bl.p);  /* losses: step-major */
+  back_Double(env, losses, bl, rc);
+  free(bs.p); free(ba.p);
+  return rc;
+}
+FN(modelsEvalCounts)(JNIEnv *env, jobject self, jlong h, jint m, jlong rowBegin, jlong rowEnd, jlongArray hingeCorrect,
+                     jdoubleArray normSquared) {
+  buf_t bc = out_Long(env, hingeCorrect), bn = out_Double(env, normSquared);
+  int rc = DSGD_ERR_NOMEM;               /* hingeCorrect(0) = hinge sum, (1) = #correct of model m */
+  if (!(bc.bad | bn.bad))
+    rc = (bc.n < 2 || bn.n < 1) ? DSGD_ERR_INVALID
+                                : dsgd_models_eval_counts(CTX(h), m, rowBegin, rowEnd, (int64_t *)bc.p, (int64_t *)bc.p + 1, bn.p);
+  back_Long(env, hingeCorrect, bc, rc);
+  back_Double(env, normSquared, bn, rc);
+  return rc;
+}
+
 /* ---- async (Hogwild) mode ---- */
 FN(asyncHostMaster)(JNIEnv *env, jobject self, jlong h, jdoubleArray w0) {
   buf_t b = in_Double(env, w0);

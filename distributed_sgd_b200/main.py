@@ -16,17 +16,35 @@ import argparse
 import json
 import os
 import time
-from typing import Optional
+from typing import Optional, Sequence
 
 import numpy as np
 
 
 def scenario(cfg, data, *, rank: int = 0, world: int = 1, device: Optional[int] = None, seed: int = 0, log=print,
-             async_concurrency: int = 64, jvm_exact: bool = False, inspect=None) -> dict:
+             async_concurrency: int = 64, jvm_exact: bool = False, inspect=None,
+             lambdas: Optional[Sequence[float]] = None, learning_rates: Optional[Sequence[float]] = None) -> dict:
     """Main.scenario (Main.scala:70-120).  inspect (tests): called as inspect("master", master) once the master exists
-    and as inspect("done", (master, state)) before the device context is released."""
+    and as inspect("done", (master, state)) before the device context is released.
+
+    lambdas / learning_rates (sync mode, one GPU, node-count 1): train every (lambda, learning rate) of their Cartesian
+    product (missing list: the configured value) as one model set (MasterSync.fit_models); the report then has one entry
+    per setting under "settings" and the index of the lowest final test loss under "best"."""
     from . import EarlyStopping, Master, Slave, SparseSVM
     from .core import Group
+    from .native import MAX_MODELS
+
+    sweep = None
+    if lambdas is not None or learning_rates is not None:
+        sweep = [(float(a), float(b)) for a in (lambdas if lambdas is not None else [cfg.lam])
+                 for b in (learning_rates if learning_rates is not None else [cfg.learning_rate])]
+        if cfg.is_async:
+            raise ValueError("--lambdas / --learning-rates train a model set in sync mode; async is set")
+        if cfg.node_count != 1 or world != 1:
+            raise ValueError(f"--lambdas / --learning-rates train a model set on one GPU with one worker: node-count is "
+                             f"{cfg.node_count} and the run has {world} processes (both must be 1)")
+        if not 1 <= len(sweep) <= MAX_MODELS:
+            raise ValueError(f"--lambdas x --learning-rates makes {len(sweep)} settings; a model set holds 1 to {MAX_MODELS}")
 
     train, test = data.split_at(int(data.n_rows * 0.8))                       # Main.scala:52
     model = SparseSVM(cfg.lam)                                                 # dimSparsity: computed by the Slave on the device
@@ -43,6 +61,23 @@ def scenario(cfg, data, *, rank: int = 0, world: int = 1, device: Optional[int] 
     report["initial_accuracy"] = master.distributed_accuracy(w0)              # Main.scala:77-78
     stop = EarlyStopping.no_improvement(patience=cfg.patience, min_delta=cfg.conv_delta, min_steps=None)
     t0 = time.perf_counter()
+    if sweep is not None:
+        states = master.fit_models(w0, cfg.max_epochs, cfg.batch_size, [a for a, _ in sweep], [b for _, b in sweep], stop)
+        report["fit_seconds"] = time.perf_counter() - t0
+        n_tr, n_te = train.n_rows, test.n_rows
+        settings = []
+        for (lam, lr), st, hist in zip(sweep, states, master.histories):
+            h, c, n2 = master.ctx.eval_counts(n_tr, n_tr + n_te, st.grad)                  # Main.scala:115-118
+            settings.append({"config": {"lam": lam, "learning_rate": lr},
+                             "history": {k: [float(x) for x in v] for k, v in hist.items()},
+                             "final_test_loss": lam * n2 + h / n_te, "final_test_accuracy": c / n_te,
+                             "final_weights_nonzero": int(np.count_nonzero(st.grad)), "updates": st.updates})
+        report["settings"] = settings
+        report["best"] = int(np.argmin([s["final_test_loss"] for s in settings]))
+        if inspect:
+            inspect("done", (master, states))
+        slave.stop()
+        return report
     if cfg.is_async:                                                          # Main.scala:82-96
         state = master.fit(w0, cfg.max_epochs, cfg.batch_size, cfg.learning_rate, stop, check_every=cfg.check_every,
                            leak_loss_coef=cfg.leaky_loss, concurrency=async_concurrency, seed=seed)
@@ -71,7 +106,13 @@ def main(argv=None) -> int:
     ap.add_argument("--seed", type=int, default=0)                            # Random.setSeed(0) (Main.scala:32)
     ap.add_argument("--jvm-exact", action="store_true",
                     help="sync mode: draw the batches from java.util.Random(seed) + Scala's Random.shuffle like the reference")
+    ap.add_argument("--lambdas", default=None,
+                    help="sync, one GPU: comma-separated lambdas; with --learning-rates, train their Cartesian product as a "
+                         "model set (at most 32 settings) and report every setting")
+    ap.add_argument("--learning-rates", default=None, help="comma-separated learning rates (see --lambdas)")
     args = ap.parse_args(argv)
+    lambdas = [float(x) for x in args.lambdas.split(",")] if args.lambdas else None
+    learning_rates = [float(x) for x in args.learning_rates.split(",")] if args.learning_rates else None
     from .utils import load_config, rcv1, synthetic_rcv1
 
     rank = int(os.environ.get("RANK", "0"))
@@ -83,7 +124,8 @@ def main(argv=None) -> int:
     cfg = load_config(args.conf)
     data = synthetic_rcv1(n_rows=args.synthetic_rows, seed=args.seed) if args.synthetic_rows else rcv1(cfg.data_path, full=cfg.full)
     report = scenario(cfg, data, rank=rank, world=world, device=local_rank, seed=args.seed,
-                      log=lambda s: print(s, flush=True), jvm_exact=args.jvm_exact)
+                      log=lambda s: print(s, flush=True), jvm_exact=args.jvm_exact, lambdas=lambdas,
+                      learning_rates=learning_rates)
     if rank == 0:
         print(json.dumps(report))
     if world > 1:

@@ -20,6 +20,7 @@ HOST_LIB_PATH = os.path.join(_PKG, "libdsgd_host.so")
 HEADER_PATH = os.path.join(os.path.dirname(_PKG), "include", "dsgd.h")
 
 UNIQUE_ID_BYTES = 128
+MAX_MODELS = 32
 IPC_HANDLE_BYTES = 64
 FLAG_ASYNC = 1
 REPLICA_SELF, REPLICA_MASTER = 0, 1
@@ -110,6 +111,11 @@ ABI = {
     "dsgd_stage_samples": [_vp, _vp, _i64],
     "dsgd_sync_steps_staged": [_vp, _i64, _i64, _i64, _f64, C.c_int],
     "dsgd_read_losses": [_vp, _vp, _i64],
+    "dsgd_models_set": [_vp, _i32, _vp, _vp, _vp],
+    "dsgd_models_shape": [_vp, C.POINTER(_i32), C.POINTER(_i32)],
+    "dsgd_models_get_weights": [_vp, _vp],
+    "dsgd_models_steps": [_vp, _vp, _i64, _i64, _vp, _vp],
+    "dsgd_models_eval_counts": [_vp, _i32, _i64, _i64, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_f64)],
     "dsgd_async_host_master": [_vp, _vp],
     "dsgd_ipc_export": [_vp, C.c_int, _vp],
     "dsgd_ipc_import": [_vp, C.c_int, _vp],
@@ -397,6 +403,46 @@ class NativeCtx:
         out = np.zeros(n_steps, dtype=np.float64)
         self._ck(self._l.dsgd_read_losses(self._h, _ptr(out), n_steps))
         return out
+
+    # -- model sets: several (lambda, learning rate) settings trained on the same draws --
+    def models_set(self, lambdas, learning_rates, w0=None):
+        """Replace the model set (an empty one frees it).  w0: [n_models, dim] or [dim] for all, or None (zeros)."""
+        lam = _arr(lambdas, np.float64)
+        lr = _arr(learning_rates, np.float64, lam.size, "learning_rates")
+        if w0 is not None:
+            w0 = np.asarray(w0, dtype=np.float64)
+            if w0.ndim == 1:
+                w0 = np.tile(_arr(w0, np.float64, self.dim, "weights"), lam.size)
+            w0 = _arr(w0, np.float64, lam.size * self.dim, "weights")
+        self._ck(self._l.dsgd_models_set(self._h, lam.size, _ptr(lam), _ptr(lr), _ptr(w0)))
+        self.n_models = lam.size
+
+    def models_shape(self) -> Tuple[int, int]:
+        n, d = C.c_int32(), C.c_int32()
+        self._ck(self._l.dsgd_models_shape(self._h, C.byref(n), C.byref(d)))
+        return n.value, d.value
+
+    def models_get_weights(self) -> np.ndarray:
+        """[n_models, dim] resident weights of the set."""
+        n, d = self.models_shape()
+        out = np.zeros(n * d, dtype=np.float64)
+        self._ck(self._l.dsgd_models_get_weights(self._h, _ptr(out)))
+        return out.reshape(n, d)
+
+    def models_steps(self, samples, n_per_step: int, n_steps: int, active=None, want_losses: bool = True):
+        """n_steps steps of every active model on the same samples; returns [n_steps, n_models] losses (NaN: frozen)."""
+        n, _ = self.models_shape()
+        samples = _arr(samples, np.int32, n_per_step * n_steps, "samples")
+        act = None if active is None else _arr(np.asarray(active, dtype=bool), np.uint8, n, "active")
+        losses = np.zeros(n_steps * n, dtype=np.float64) if want_losses else None
+        self._ck(self._l.dsgd_models_steps(self._h, _ptr(samples), n_per_step, n_steps, _ptr(act), _ptr(losses)))
+        return None if losses is None else losses.reshape(n_steps, n)
+
+    def models_eval_counts(self, m: int, row_begin: int, row_end: int) -> Tuple[int, int, float]:
+        """eval_counts for model m's resident weights."""
+        h, c, n2 = C.c_int64(), C.c_int64(), C.c_double()
+        self._ck(self._l.dsgd_models_eval_counts(self._h, m, row_begin, row_end, C.byref(h), C.byref(c), C.byref(n2)))
+        return h.value, c.value, n2.value
 
     # -- async --
     def async_host_master(self, w0):

@@ -172,6 +172,31 @@ int dsgd_sync_steps_staged(dsgd_ctx *ctx, int64_t first, int64_t n_per_step, int
                            int want_losses);
 int dsgd_read_losses(dsgd_ctx *ctx, double *losses_out, int64_t n_steps);
 
+/* ---- model sets: several SparseSVMs, each with its own lambda and learning rate, trained on the SAME batch draws.
+ *      The reference trains one `new SparseSVM(config.lambda, ...)` per run (Main.scala:68) with the batch loop of
+ *      Master.fit (core/Master.scala:179-198); a lambda / learning-rate sweep reruns everything.  A model set runs the
+ *      steps of all its models in one persistent kernel per call: they share the sample ids, the row loads, the launch
+ *      and one grid barrier per step.  One GPU and one worker per step (world == 1, the default dsgd_set_workers);
+ *      at most 32 samples per SM and step.  Each model follows exactly the arithmetic of dsgd_sync_steps with its own
+ *      lambda and lr.  Model-set calls leave the ctx's resident weights (dsgd_get_weights) untouched. */
+#define DSGD_MAX_MODELS 32
+/* Replace the ctx's model set (n_models == 0 frees it).  lambda, lr: [n_models]; lambda finite and >= 0, lr finite.
+ * w0: [n_models * dim] initial weights, model-major, or NULL (zeros). */
+int dsgd_models_set(dsgd_ctx *ctx, int32_t n_models, const double *lambda, const double *lr, const double *w0);
+/* n_models of the current set (0: none) and dim, so that a binding can size its buffers. */
+int dsgd_models_shape(const dsgd_ctx *ctx, int32_t *n_models, int32_t *dim);
+/* w_out: [n_models * dim], model-major. */
+int dsgd_models_get_weights(dsgd_ctx *ctx, double *w_out);
+/* n_steps steps of every active model on the same samples (n_steps * n_per_step ids, step-major, like dsgd_sync_steps).
+ * active: [n_models], non-zero = takes part, or NULL (all); a frozen model keeps its weights bit for bit.
+ * losses_out: [n_steps * n_models] step-major (SparseSVM.loss at the pre-step weights; NaN for frozen models) or NULL.
+ * Several calls in a row continue one trajectory per model. */
+int dsgd_models_steps(dsgd_ctx *ctx, const int32_t *samples, int64_t n_per_step, int64_t n_steps, const uint8_t *active,
+                      double *losses_out);
+/* dsgd_eval_counts over rows [row_begin, row_end) for model m's resident weights. */
+int dsgd_models_eval_counts(dsgd_ctx *ctx, int32_t m, int64_t row_begin, int64_t row_end, int64_t *hinge_sum,
+                            int64_t *correct, double *norm_squared);
+
 /* ---- async (Hogwild) mode.  Every worker keeps its own weight replica (core/Slave.scala:30) and pushes each
  *      delta to every peer replica and to the master's replica (core/Slave.scala:101-105).  Here replicas are
  *      reached by ADDRESS over NVLink: a rank exports its replica, the host transports the handle, peers import
