@@ -328,9 +328,13 @@ __global__ void __launch_bounds__(256) k_repack(const int64_t *__restrict__ row_
     for (int64_t k = lane; k < de - db; k += 32) {
       uint2 pr;
       if (k < len) {
+        // a value the Sparse constructor drops (|x| <= 1e-20, math/Sparse.scala:108-118) is stored as +0: every fp64
+        // consumer applies filt(x) first and sees the same absent key, and the fp32 dot of the streaming pass no longer
+        // adds a product the fp64 arithmetic never forms (its rounding band, dsgd_stream.cuh, relies on this)
+        const double xv = filt((double)val[sb + k]);
         pr.x = (uint32_t)col[sb + k];
-        pr.y = __float_as_uint(val[sb + k]);
-        asum += fabs((double)val[sb + k]);
+        pr.y = __float_as_uint((float)xv);
+        asum += fabs(xv);
       } else {
         pr.x = len > 0 ? (uint32_t)col[se - 1] : 0u;
         pr.y = 0u;

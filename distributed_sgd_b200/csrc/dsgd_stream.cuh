@@ -22,12 +22,20 @@
 //     are back to back in the pair array -- so its four loads leave before the row-end masks are even computed.
 //   * Blocks are dealt dynamically (one atomic per block, requested a block ahead); the last fifth of a pass goes out in
 //     blocks of half the size so the warps run dry together.
-//   * Exactness against the fp64 arithmetic of the reference: the fp32 result differs from x.w by at most
-//       (D + 1) * 2^-24 * max|w| * sum|x|,   D = units/32 + 9 roundings on the longest add chain, + 1 for rounding w
-//     (first-order bound, 1.5x slack); sum|x| per row is computed once when the rows are loaded (k_repack, rounded
-//     up, stored with the label in its sign bit: one 4-byte load per row).  Rows whose |dot| is inside that band are
-//     recomputed with the fp64 weights from L2 after the block's stream, so every prediction and gate decision is
-//     that of the fp64 arithmetic (tests/test_gpu_parity.py::test_streaming_exact_fallback_decides_like_fp64).
+//   * Exactness against the fp64 arithmetic of the reference.  That arithmetic sums filt(x_j * w_j): values with
+//     |x| <= 1e-20 never enter a row (math/Sparse.scala:108-118; k_repack stores them as 0 and leaves them out of sum|x|),
+//     and products with |x w| <= 1e-20 are dropped.  The fp32 result differs from that sum by at most
+//       (D + 1) * 2^-24 * max|w| * sum|x|      relative rounding: D = units/32 + 9 roundings on the longest add chain,
+//                                              + 1 for rounding w to fp32 (first-order bound)
+//     + 2^-150 * sum|x|                        absolute rounding of weights that become fp32 subnormals (or 0)
+//     + 1e-20 * pairs                          the products the filter drops; this term also covers the absolute
+//                                              rounding of subnormal fp32 products and sums (2^-150 per operation)
+//     and the threshold is that bound with 1.5x slack, computed in fp64 so that no term underflows (an fp32 band of
+//     2^-24 * max|w| is subnormal below max|w| ~ 1e-31); a dot that overflowed fp32 is never trusted.  sum|x| per row is
+//     computed once when the rows are loaded (k_repack, rounded up, stored with the label in its sign bit: one 4-byte
+//     load per row).  Rows whose |dot| is inside the band are recomputed with the fp64 weights from L2 after the block's
+//     stream, so every prediction and gate decision is that of the fp64 arithmetic
+//     (tests/test_gpu_parity.py::test_streaming_exact_fallback_decides_like_fp64, tests/test_gpu_edge_regimes.py).
 //   * Scatter (gradient): rows that pass the gate are re-walked after the block's stream (their units are in
 //     L1/L2) and y*x goes to g with fp64 REDs.  On trained weights few rows pass (the misclassified ones) and the pass
 //     runs at the streaming rate; on untrained weights every row passes and the fp64 RED rate at L2 bounds it
@@ -142,7 +150,7 @@ __global__ void __launch_bounds__(kStreamThreads, 1) k_stream_rows(const StreamP
 #pragma unroll
     for (int i = 0; i < kStreamThreads / 32; ++i) wmax = fmaxf(wmax, s_wmax[i]);
   }
-  const float band_scale = 1.5f * 5.9604645e-8f * wmax;   // 1.5 * 2^-24 * max|w|
+  const double band_rel = 1.5 * 0x1p-24 * (double)wmax;   // 1.5 * 2^-24 * max|w|, in fp64: no underflow for any fp32 wmax
   // one gradient entry (SparseSVM.scala:26-29): a reduction without a return value
   auto scatter_one = [&](uint32_t col, double gv) {
     if (gv != 0.0) red_add_f64(&p.g[col], gv);
@@ -264,8 +272,12 @@ __global__ void __launch_bounds__(kStreamThreads, 1) k_stream_rows(const StreamP
       do_scatter = kScatter && (pr != y);
     };
     if (valid) {
-      const float thresh = band_scale * fabsf(ya) * (float)((len >> 5) + 10) + 1e-30f;
-      if (!(fabsf(dot_mine) > thresh)) need_exact = true;   // also catches NaN
+      // the band of the header comment: relative rounding (D + 1) * 2^-24 * max|w| * sum|x|, absolute rounding of fp32
+      // weights below 2^-126 (2^-150 per unit of sum|x|), and the products of at most 1e-20 that the fp64 arithmetic drops
+      // (<= 2 * len pairs); all with 1.5x slack, in fp64 so that no term underflows
+      const double thresh = (double)fabsf(ya) * (band_rel * (double)((len >> 5) + 10) + 1.5 * 0x1p-150) + 3e-20 * (double)len;
+      const float ad = fabsf(dot_mine);
+      if (!((double)ad > thresh && ad <= 3.4028235e38f)) need_exact = true;   // also catches NaN and an fp32 overflow
       else finalize(dot_mine > 0.f ? -1 : 1);
     }
     // ---- exact recomputation of the rows the fp32 sign could not decide ----

@@ -39,25 +39,43 @@ def start_weights(rng, dim, M):
     return w0
 
 
-def check_against_oracle(orc, w0, idx, batch, losses, W, lams=LAMS, lrs=LRS):
+def check_against_oracle(orc, w0, idx, batch, losses, W, lams=LAMS, lrs=LRS, atol=1e-15):
+    """atol None: 1e-13 * max|w| -- fp64 sums in another order whose result cancels to far below the summands keep an
+    absolute error at the summands' scale (as in smoke()); needed once weights reach O(1) or c is large."""
     steps = idx.shape[0]
     for m, (lam, lr) in enumerate(zip(lams, lrs)):
         w_ref, l_ref = oracle_for(orc, lam).sync_steps(w0[m], idx.reshape(-1), [batch], lr, n_steps=steps)
         np.testing.assert_allclose(losses[:, m], l_ref, rtol=RTOL, err_msg=f"model {m}")
         assert (W[m] == 0).tolist() == (w_ref == 0).tolist(), f"model {m}: weight supports differ"
-        np.testing.assert_allclose(W[m], w_ref, rtol=1e-11, atol=1e-15, err_msg=f"model {m}")
+        np.testing.assert_allclose(W[m], w_ref, rtol=1e-11, err_msg=f"model {m}",
+                                   atol=1e-13 * float(np.abs(w_ref).max()) if atol is None else atol)
 
 
-@pytest.mark.parametrize("batch,steps", [(1, 40), (16, 60), (256, 30)])
-def test_model_set_trajectories(synth, batch, steps):
-    rng = np.random.default_rng(100 + batch)
+def settings_for(M):
+    """M (lambda, learning rate) settings: the five above for M = 5, else lambda 0 then 1e-6 .. 1e-2 geometrically with
+    learning rates 1 .. 0.05 evenly (the largest lambda with the smallest rate: lambda 1e-2 at rate 1 diverges)."""
+    if M == len(LAMS):
+        return LAMS, LRS
+    return [0.0] + list(np.geomspace(1e-6, 1e-2, M - 1)), list(np.linspace(1.0, 0.05, M))
+
+
+@pytest.mark.parametrize("batch,steps,M", [
+    pytest.param(1, 40, 5, id="1-40"), pytest.param(16, 60, 5, id="16-60"), pytest.param(256, 30, 5, id="256-30"),
+    # models 8-31 are read through the shuffle groups 1-3 of acc_read_models and use the per-model slots k >= 8
+    pytest.param(256, 20, 8, id="256-20-M8"), pytest.param(256, 20, 9, id="256-20-M9"),
+    pytest.param(256, 20, 16, id="256-20-M16"), pytest.param(256, 20, 32, id="256-20-M32"),
+    pytest.param(1, 20, 32, id="1-20-M32")])
+def test_model_set_trajectories(synth, batch, steps, M):
+    rng = np.random.default_rng(100 + batch + (M if M != len(LAMS) else 0))
+    lams, lrs = settings_for(M)
     ctx, orc = make_pair(synth, lam=1e-5, n_train=4800)
     idx = draws(rng, 4800, batch, steps)
-    w0 = start_weights(rng, synth.dim, len(LAMS))
-    ctx.models_set(LAMS, LRS, w0)
+    w0 = start_weights(rng, synth.dim, M)
+    ctx.models_set(lams, lrs, w0)
     losses = ctx.models_steps(idx.reshape(-1), batch, steps)
-    assert losses.shape == (steps, len(LAMS))
-    check_against_oracle(orc, w0, idx, batch, losses, ctx.models_get_weights())
+    assert losses.shape == (steps, M)
+    check_against_oracle(orc, w0, idx, batch, losses, ctx.models_get_weights(), lams, lrs,
+                         atol=1e-15 if M == len(LAMS) else None)
     ctx.close()
 
 
